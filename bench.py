@@ -29,8 +29,10 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 
 N_TABLES = 4096
+DUMP_OBS_ROWS = 256  # --dump-outputs: observation rows kept (256 x 137,632 B = 35 MB)
 SEED_START = (10000, 0x2000)  # mortal/player.py:67
 OBS_BYTES = 1012 * 34 * 4
 MASK_BYTES = 46
@@ -301,6 +303,61 @@ class HostNetEngine:
         return self.e.react_batch(obs, masks, invisible_obs)
 
 
+class LastStepRecorder:
+    """The DeviceEngine as the arena drives it, plus a device copy of one cycle's exchange: the rows the engine is handed
+    (observations, legal masks, and the rows' table / seat from the environment) and the actions and Q-values it returns.
+    Armed for the last timed cycle by the bench's cycle hook (--dump-outputs)."""
+
+    def __init__(self, engine):
+        self.e = engine
+        for attr in ("engine_type", "name", "version", "is_oracle", "enable_quick_eval", "enable_rule_based_agari_guard"):
+            setattr(self, attr, getattr(engine, attr))
+        self.env = None
+        self.last = None
+
+    def react_device(self, obs, masks, invisible_obs=None):
+        return self.e.react_device(obs, masks)
+
+    def react_static(self, obs_buf, masks_buf, nr):
+        a, q = self.e.react_static(obs_buf, masks_buf, nr)
+        if self.env is not None:
+            self.last = dict(obs=obs_buf[:nr].clone(), masks=masks_buf[:nr].clone(), actions=a.clone(), q_values=q.clone(),
+                             row_table=self.env.row_table[:nr].clone(), row_seat=self.env.row_seat[:nr].clone())
+            self.env = None
+        return a, q
+
+
+def dump_outputs(out_dir, last):
+    """Write one recorded cycle as DIR/<name>.npy (float32 / float64). Rows are sorted by (table, seat byte): the environment
+    appends decision rows through an atomic counter, so their order differs from run to run while their content does not.
+    The observations are a fixed seeded sample of DUMP_OBS_ROWS of the sorted rows (obs_sample_rows: their positions).
+    The engine returns -inf as the Q-value of an illegal action; q_values holds 0 there (masks says which entries are legal),
+    so every written value is finite and a non-finite one is an error."""
+    import numpy as np
+    import torch
+
+    if last is None:
+        raise SystemExit("bench.py --dump-outputs: the last timed step had no decision rows to record")
+    order = torch.argsort(last["row_table"].long() * 8 + last["row_seat"].long())
+    n = int(order.numel())
+    pick = np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_OBS_ROWS), replace=False))
+    arrays = {
+        "row_table": last["row_table"][order].double(),
+        "row_seat": last["row_seat"][order].double(),  # seat | 4 on kan-select rows
+        "masks": last["masks"][order].float(),
+        "actions": last["actions"][order].double(),
+        "q_values": last["q_values"][order].float().masked_fill(~last["masks"][order], 0.0),
+        "obs_sample": last["obs"][order[torch.from_numpy(pick).to(order.device)]].float(),
+        "obs_sample_rows": torch.from_numpy(pick).double(),
+    }
+    for name, t in arrays.items():
+        if not bool(torch.isfinite(t).all()):
+            raise SystemExit(f"bench.py --dump-outputs: {name} of the last timed step holds a non-finite value")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -413,6 +470,8 @@ def run_ours(args):
             if c in (n_warm, n_warm + n_timed):
                 torch.cuda.synchronize()
                 marks[c] = (time.perf_counter(), state.total_steps(), rows())
+            if c == n_warm + n_timed - 1 and isinstance(agent, LastStepRecorder):
+                agent.env = state.parts[0].env
 
         arena.cycle_hook = hook
         # same tables as the other loops: rank r starts at seed_start + 1024 r
@@ -433,9 +492,13 @@ def run_ours(args):
     a_nn_ms = sum(e[1].elapsed_time(e[2]) for e in a_split) / K
     ea[0].close()
     barrier()
-    av = run_arena(engine, W, K)  # the headline `value`: the same workload through the arena (pipelined half-batches)
+    recorder = LastStepRecorder(engine) if args.dump_outputs else None
+    av = run_arena(recorder or engine, W, K)  # the headline `value`: the same workload through the arena (pipelined half-batches)
     barrier()
     clocks = sampler.stop()
+    if recorder is not None and rank == 0:
+        dump_outputs(args.dump_outputs, recorder.last)
+        recorder.last = None
 
     # -------- loop B: env only (test policy on device, no host sync); B2 = the same with the single-player block off
     ea = fresh_env()
@@ -758,6 +821,9 @@ def main():
     ap.add_argument("--no-e2e-net", action="store_true")
     ap.add_argument("--no-algo-1m", action="store_true", help="skip BASELINE configs[2] (shanten / agari at 1M hands)")
     ap.add_argument("--no-encode-64k", action="store_true", help="skip the BASELINE configs[3] encode measurement (27 GB obs buffer)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed `value` path computed in its last timed step (observation sample, masks, "
+                         "actions, Q-values, row ids) as DIR/<name>.npy; inputs are seeded, so runs with the same arguments compare")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3

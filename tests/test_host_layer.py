@@ -354,56 +354,6 @@ def test_arena_host_protocol_loop_on_emulated_env_fail_fast():
     assert (ref["scores"] == arena.last_results["scores"]).all() and (ref["ranks"] == arena.last_results["ranks"]).all()
 
 
-def test_reference_mortal_engine_and_model_drop_in_unchanged():
-    """north_star: "mortal/train.py and mortal/engine.py drop in unchanged". The reference's OWN, unmodified mortal/engine.py
-    (MortalEngine) and mortal/model.py (Brain, DQN) are imported from /root/reference against the `libriichi` module this repo
-    installs, and drive libriichi.arena.OneVsThree.py_vs_py exactly like mortal/player.py:60-69 does (host-emulated environment:
-    this container has no GPU). The recorded decisions replay in the oracle to the same scores / rankings. Skipped where the
-    reference tree is absent (the GPU box)."""
-    import importlib
-    import sys
-
-    import pytest
-
-    ref_dir = "/root/reference/mortal"
-    if not os.path.isdir(ref_dir):
-        pytest.skip("reference tree not present")
-    import torch
-
-    import mortal_b200.libriichi as lr
-
-    lr.install()
-    sys.path.insert(0, ref_dir)
-    try:
-        for name in ("model", "engine"):
-            sys.modules.pop(name, None)
-        ref_model = importlib.import_module("model")
-        ref_engine = importlib.import_module("engine")
-    finally:
-        sys.path.remove(ref_dir)
-    assert ref_model.__file__.startswith(ref_dir) and ref_engine.__file__.startswith(ref_dir)
-    from libriichi.arena import OneVsThree
-
-    torch.manual_seed(0)
-    mk = lambda name: ref_engine.MortalEngine(ref_model.Brain(version=4, conv_channels=16, num_blocks=1).eval(),
-                                              ref_model.DQN(version=4).eval(), is_oracle=False, version=4,
-                                              device=torch.device("cpu"), enable_amp=False, enable_quick_eval=True,
-                                              enable_rule_based_agari_guard=False, name=name)
-    arena = _emul_arena(OneVsThree)
-    arena.record_decisions = True
-    rankings = arena.py_vs_py(challenger=mk("challenger"), champion=mk("champion"), seed_start=(10000, 0x2000), seed_count=1)
-    assert sum(rankings) == 4
-    nonces = np.repeat(np.arange(10000, 10001, dtype=np.uint64), 4)
-    keys = np.full(4, 0x2000, dtype=np.uint64)
-    ref = O.run_replay(nonces, keys, arena.last_decisions, quick_eval=True, mask_bits=arena.last_decision_masks)
-    got = arena.last_results
-    assert (ref["scores"] == got["scores"]).all() and (ref["ranks"] == got["ranks"]).all() and (ref["steps"] == got["steps"]).all()
-    hist = [0, 0, 0, 0]
-    for i in range(4):
-        hist[int(ref["ranks"][i, i % 4])] += 1
-    assert hist == rankings
-
-
 def test_arena_feeds_oracle_engines_the_invisible_observation():
     """agent/mortal.rs:253-255, 137-146: an engine with is_oracle=True receives invisible_obs (list of (217, 34) arrays, one per row)
     next to obs and masks; an ordinary engine receives None. Checked on the host-emulated environment: the other seats' hand

@@ -1,6 +1,8 @@
 """The shanten and agari lookup tables are generated from first principles (tools/gen_shanten_tables.cc,
-tools/gen_agari_table.py); this pins the generators."""
-import gzip
+tools/gen_agari_table.py); this pins the generators. libriichi's own data files are held in tests/golden/ref_tables.json
+as a digest of their whole content plus a sample of rows (written by tools/extract_ref_fixtures.py)."""
+import hashlib
+import json
 import os
 import sys
 
@@ -9,7 +11,8 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tools"))
-REF = "/root/reference/libriichi/src/algo/data"
+with open(os.path.join(ROOT, "tests", "golden", "ref_tables.json")) as _f:
+    REF_TABLES = json.load(_f)
 
 
 @pytest.fixture(scope="module")
@@ -42,11 +45,13 @@ def test_generated_rows_known_answers(generated):
     assert nibbles(jihai[idx([3, 2, 1, 0, 0, 0, 0])]) == [0, 0, 1, 3, 6, 0, 0, 2, 5, 8]
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box): generator is pinned in the dev container")
 def test_generated_tables_equal_reference_data(generated):
     for name in ("shanten_suhai.bin", "shanten_jihai.bin"):
-        with gzip.open(os.path.join(REF, name + ".gz"), "rb") as f:
-            assert f.read() == generated[name], name
+        ref, raw = REF_TABLES[name], generated[name]
+        rows = np.frombuffer(raw, dtype=np.uint8).reshape(-1, 5)
+        for i, want in ref["sample_rows"].items():
+            assert rows[int(i)].tobytes().hex() == want, (name, i)
+        assert len(raw) == ref["bytes"] and hashlib.sha256(raw).hexdigest() == ref["sha256"], name
 
 
 def test_installed_tables_are_the_generated_ones(generated):
@@ -89,13 +94,14 @@ def test_agari_table_known_answers(agari_table):
             assert (d & 7) + ((d >> 3) & 7) <= 4
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present (GPU box): generator is pinned in the dev container")
 def test_agari_table_equals_reference_data(agari_table):
-    import gen_agari_table as g
+    from extract_ref_fixtures import agari_digest
 
-    with gzip.open(os.path.join(REF, "agari.bin.gz"), "rb") as f:
-        ref = g.parse(f.read())
-    assert ref == agari_table  # key -> ordered list of divs; the record order of the file is not content (agari.rs:22-51)
+    # key -> ordered list of divs; the record order of the file is not content (agari.rs:22-51)
+    ref = REF_TABLES["agari.bin"]
+    for key, divs in ref["sample"].items():
+        assert agari_table.get(int(key, 16)) == divs, key
+    assert len(agari_table) == ref["keys"] and agari_digest(agari_table) == ref["sha256"]
 
 
 def test_installed_agari_table_is_the_generated_one(agari_table):
