@@ -236,6 +236,26 @@ int mjx_nn_block_tail_bf16(const void* y, const void* x, const float* w1, const 
                            const float* scale, const float* bias, void* gate_scratch /* bf16 [batch, channels] */, void* x_out,
                            void* a_out, int batch, int length, int channels, int hidden, void* stream);
 
+/* mjx_nn_obs_to_nhwc_bf16 of a gathered batch: output row i is observation rows[i] for i < *count_dev, zeros for the rest of
+ * `batch` (rows, count_dev: device int32). */
+int mjx_nn_obs_rows_to_nhwc_bf16(const float* obs, const int* rows, const int* count_dev, void* out, int batch, int channels, int length,
+                                 int channels_padded, void* stream);
+
+/* ---- action selection on the device path (mortal/engine.py MortalEngine._react_batch + mortal/model.py DQN.forward) --------------
+ * Batch row i < min(*count_dev, n_max) is environment row r = rows[i] (rows NULL: r = i); v f32 [n] and a f32 [n, 46] with row strides.
+ * Writes q_out[r] (dueling Q, -inf on illegal actions per masks[r]), actions[r] (int64) and greedy[r] (uint8, optional): the argmax
+ * (lowest index on ties), or with probability epsilon a draw from softmax(q / temp) over the top-p nucleus of the legal actions.
+ * Randomness: Philox4x32-10 with key `seed` and counter (table_offset + row_table[r], row_step[r], row_seat[r]), so a decision's
+ * draw does not depend on the order of the rows. */
+int mjx_select_actions(const float* v, long long v_stride, const float* a, long long a_stride, const int* rows, const int* count_dev,
+                       int n_max, const void* masks, const int* row_table, const uint32_t* row_step, const uint8_t* row_seat,
+                       unsigned long long seed, int table_offset, float epsilon, float temp, float top_p, int64_t* actions,
+                       float* q_out, uint8_t* greedy, void* stream);
+/* Stable split of the step's *count_dev rows by agent_of[row_table * 4 + (row_seat & 3)] (0 or 1): rows0 / rows1 get the row indices
+ * in order, counts[0..1] (device int32) their numbers. One CTA. */
+int mjx_split_rows(const int* row_table, const uint8_t* row_seat, const int* count_dev, const uint8_t* agent_of, int* rows0, int* rows1,
+                   int* counts, void* stream);
+
 /* ---- standalone kernels (BASELINE configs 3/4) ------------------------------------------------ */
 /* algo/shanten.rs:138-150 calc_all: tiles_dev uint8 [n,34], len_div3_dev uint8 [n] -> int8 [n]. */
 int mjx_shanten(const uint8_t* tiles_dev, const uint8_t* len_div3_dev, int8_t* out_dev, int n, void* stream);

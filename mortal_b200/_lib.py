@@ -69,6 +69,11 @@ SYMBOLS = {
     "mjx_nn_gate_residual_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "mjx_nn_obs_to_nhwc_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "mjx_nn_block_tail_bf16": (C.c_int, [C.c_void_p] * 11 + [C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "mjx_nn_obs_rows_to_nhwc_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]),
+    "mjx_select_actions": (C.c_int, [C.c_void_p, C.c_longlong, C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_ulonglong, C.c_int, C.c_float, C.c_float, C.c_float,
+                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mjx_split_rows": (C.c_int, [C.c_void_p] * 8),
     "mjx_env_create_replay": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p,
                                         C.c_void_p, C.c_longlong, C.c_void_p, C.c_int, C.c_int]),
     "mjx_env_replay_trust_seeds": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),

@@ -12,6 +12,7 @@
 #include "mjx_invisible.cuh"
 #include "mjx_state.cuh"
 #include "mjx_nn.cuh"
+#include "mjx_select.cuh"
 #include "mjx_tables_host.h"
 
 using namespace mjx;
@@ -1394,7 +1395,48 @@ int mjx_nn_obs_to_nhwc_bf16(const float* obs, void* out, int batch, int channels
     const size_t smem = (size_t)mjx_nn::NHWC_TC * (length + 1) * sizeof(float);
     const long long grid = (long long)batch * (channels_padded / mjx_nn::NHWC_TC);
     if (grid > 0x7fffffffLL) return fail(MJX_ERR_ARG, "mjx_nn_obs_to_nhwc_bf16: batch too large");
-    mjx_nn::k_obs_to_nhwc<<<(int)grid, 256, smem, (cudaStream_t)stream>>>(obs, (__nv_bfloat16*)out, channels, length, channels_padded);
+    mjx_nn::k_obs_to_nhwc<false><<<(int)grid, 256, smem, (cudaStream_t)stream>>>(obs, (__nv_bfloat16*)out, channels, length, channels_padded,
+                                                                          nullptr, nullptr);
+    CU(cudaGetLastError());
+    return MJX_OK;
+}
+int mjx_nn_obs_rows_to_nhwc_bf16(const float* obs, const int* rows, const int* count, void* out, int batch, int channels, int length,
+                                 int channels_padded, void* stream) {
+    if (!obs || !rows || !count || !out || batch <= 0 || channels <= 0 || length <= 0 || length > 128 || channels_padded < channels ||
+        channels_padded % mjx_nn::NHWC_TC)
+        return fail(MJX_ERR_ARG, "mjx_nn_obs_rows_to_nhwc_bf16: bad arguments (channels_padded a multiple of 64, length <= 128)");
+    if (!g_ready) return fail(MJX_ERR_STATE, "mjx_nn_*: call mjx_init first");
+    const size_t smem = (size_t)mjx_nn::NHWC_TC * (length + 1) * sizeof(float);
+    const long long grid = (long long)batch * (channels_padded / mjx_nn::NHWC_TC);
+    if (grid > 0x7fffffffLL) return fail(MJX_ERR_ARG, "mjx_nn_obs_rows_to_nhwc_bf16: batch too large");
+    mjx_nn::k_obs_to_nhwc<true><<<(int)grid, 256, smem, (cudaStream_t)stream>>>(obs, (__nv_bfloat16*)out, channels, length, channels_padded,
+                                                                         rows, count);
+    CU(cudaGetLastError());
+    return MJX_OK;
+}
+int mjx_select_actions(const float* v, long long v_stride, const float* a, long long a_stride, const int* rows, const int* count,
+                       int n_max, const void* masks, const int* row_table, const uint32_t* row_step, const uint8_t* row_seat,
+                       unsigned long long seed, int table_offset, float epsilon, float temp, float top_p, int64_t* actions,
+                       float* q_out, uint8_t* greedy, void* stream) {
+    if (!v || !a || !count || !masks || !row_table || !row_step || !row_seat || !actions || !q_out || n_max < 0 || a_stride < 46 ||
+        v_stride < 1 || epsilon < 0.f || epsilon > 1.f || (epsilon > 0.f && !(temp > 0.f)))
+        return fail(MJX_ERR_ARG, "mjx_select_actions: bad arguments");
+    if (n_max == 0) return MJX_OK;
+    mjx_sel::SelectArgs A{v, v_stride, a, a_stride, rows, count, n_max, (const uint8_t*)masks, row_table, row_step, row_seat,
+                          (uint32_t)seed, (uint32_t)(seed >> 32), table_offset, epsilon, epsilon > 0.f ? 1.f / temp : 1.f, top_p,
+                          actions, q_out, greedy};
+    const int warps_per_cta = 8;
+    const int grid = std::max(1, std::min((n_max + warps_per_cta - 1) / warps_per_cta, g_sm_count * 16));
+    mjx_sel::k_select_actions<<<grid, warps_per_cta * 32, 0, (cudaStream_t)stream>>>(A);
+    CU(cudaGetLastError());
+    return MJX_OK;
+}
+int mjx_split_rows(const int* row_table, const uint8_t* row_seat, const int* count, const uint8_t* agent_of, int* rows0, int* rows1,
+                   int* counts, void* stream) {
+    if (!row_table || !row_seat || !count || !agent_of || !rows0 || !rows1 || !counts)
+        return fail(MJX_ERR_ARG, "mjx_split_rows: bad arguments");
+    mjx_sel::k_split_rows<<<1, mjx_sel::SPLIT_THREADS, 0, (cudaStream_t)stream>>>(row_table, row_seat, count, agent_of, rows0, rows1,
+                                                                                 counts);
     CU(cudaGetLastError());
     return MJX_OK;
 }

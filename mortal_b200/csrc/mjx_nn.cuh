@@ -199,14 +199,22 @@ __global__ void __launch_bounds__(256) k_gate_residual_mish(const Vec8* __restri
 // per channel) -> bf16 channels-last [batch, length, cpad] with the channel count padded with zeros to a multiple of 64, which is
 // what the stem convolution's implicit GEMM wants (PyTorch + cuDNN otherwise run a cast, a layout copy and two padding kernels).
 // One CTA = 64 channels of one observation through a shared-memory tile.
+// GATHER: output row b is observation rows[b] for b < *count and all zeros past it (a per-engine batch converted straight from the
+// environment's observation buffer; the zero rows pad the batch to the bucket a CUDA graph was captured for).
 constexpr int NHWC_TC = 64;
+template <bool GATHER>
 __global__ void __launch_bounds__(256) k_obs_to_nhwc(const float* __restrict__ obs, __nv_bfloat16* __restrict__ out, int channels, int length,
-                                                     int cpad) {
+                                                     int cpad, const int* __restrict__ rows, const int* __restrict__ count) {
     extern __shared__ float tile[];  // [NHWC_TC][length + 1]
     const int chunks = cpad / NHWC_TC;
     const int b = blockIdx.x / chunks, c0 = (blockIdx.x - b * chunks) * NHWC_TC;
-    const int nc = max(0, min(NHWC_TC, channels - c0));  // real channels in this chunk
-    const float* src = obs + ((size_t)b * channels + c0) * length;
+    int nc = max(0, min(NHWC_TC, channels - c0));  // real channels in this chunk
+    size_t src_row = b;
+    if constexpr (GATHER) {
+        if (b < *count) src_row = (size_t)rows[b];
+        else nc = 0;
+    }
+    const float* src = obs + (src_row * channels + c0) * length;
     const int pitch = length + 1;
     for (int i = threadIdx.x; i < nc * length; i += blockDim.x) {
         const int c = i / length, l = i - c * length;

@@ -5,6 +5,7 @@ on-device actions, with the selection semantics of mortal/engine.py:43-94 (maske
 epsilon-Boltzmann with top-p). Any object following the reference's duck-typed protocol
 (agent/mortal.rs:54-74, 126-152: `engine_type == 'mortal'`, `react_batch(list[np], list[np], None)`)
 still works through `HostProtocolEngine`, which pays the device->host->device round trip the reference pays.
+`ReferenceEngine` puts Mortal's own MortalEngine (versions 2-4) on the device path when the arena is told to adopt it.
 """
 from __future__ import annotations
 
@@ -160,3 +161,93 @@ class HostProtocolEngine:
         actions, q, _, _ = self.engine.react_batch(list(obs_h), list(masks_h), inv)
         dev = obs.device
         return torch.as_tensor(actions, dtype=torch.int64, device=dev), torch.as_tensor(q, dtype=torch.float32, device=dev)
+
+
+class ReferenceEngine:
+    """The device path for an unmodified mortal/engine.py MortalEngine holding a version 2, 3 or 4 Brain / DQN.
+
+    Reads only the attributes MortalEngine.__init__ sets and never touches the caller's modules: `refresh()` builds an inference
+    copy through their state_dict() and mortal_b200.checkpoint (mortal/train.py keeps training the same modules between plays, so
+    the arena calls it at every py_vs_py). `enable_amp=True` runs the BN-folded bf16 fused path (MortalEngine autocasts to fp16
+    instead), `enable_amp=False` fp32 channels-last convolutions. Per (observation buffer, batch bucket) one CUDA graph covers the
+    stem conversion of the engine's rows, the network, the Q head and k_select_actions (csrc/mjx_select.cuh), greedy or
+    epsilon-Boltzmann / top-p alike. The sampling seed is drawn from torch's default generator at construction, so
+    torch.manual_seed makes sampled self-play repeat exactly."""
+
+    engine_type = "mortal"
+    ATTRS = ("version", "is_oracle", "enable_amp", "enable_quick_eval", "enable_rule_based_agari_guard", "name",
+             "boltzmann_epsilon", "boltzmann_temp", "top_p")
+
+    @staticmethod
+    def eligible(engine, device: int) -> bool:
+        """MortalEngine-shaped (engine_type 'mortal', brain, dqn), version 2-4, not an oracle, on CUDA device `device`"""
+        if hasattr(engine, "react_device") or getattr(engine, "engine_type", None) != "mortal":
+            return False
+        if not (hasattr(engine, "brain") and hasattr(engine, "dqn")):
+            return False
+        dev = getattr(engine, "device", None)
+        return (getattr(engine, "version", None) in (2, 3, 4) and not getattr(engine, "is_oracle", False)
+                and isinstance(dev, torch.device) and dev.type == "cuda" and (dev.index or 0) == int(device))
+
+    def __init__(self, engine):
+        self.engine = engine
+        for attr in self.ATTRS:
+            setattr(self, attr, getattr(engine, attr))
+        self.device = torch.device("cuda", engine.device.index or 0)
+        self.seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+        self.brain = self.dqn = None
+        self._graphs = {}
+        self.graph_captures = 0
+        self.graph_replays = 0
+
+    @torch.no_grad()
+    def refresh(self):
+        from . import _lib
+        from .checkpoint import load_reference_state_dicts
+
+        _lib.init(self.device.index)
+        brain, dqn = load_reference_state_dicts(self.engine.brain.state_dict(), self.engine.dqn.state_dict(), self.version)
+        self.brain = brain.to(self.device).eval().prepare_fast(torch.bfloat16 if self.enable_amp else None)
+        self.dqn = dqn.to(self.device).eval()
+        self._graphs = {}
+
+    def _forward_select(self, obs_buf, env, rows, count, nb, table_offset, actions, q_out, greedy):
+        from . import nn_ops
+
+        if self.enable_amp:
+            if rows is None:
+                x = nn_ops.obs_to_nhwc(obs_buf[:nb], self.brain._cpad)
+            else:
+                x = nn_ops.obs_rows_to_nhwc(obs_buf, rows, count, nb, self.brain._cpad)
+            phi = self.brain.forward_fast_nhwc(x).float()
+        else:
+            phi = self.brain.forward_fast(obs_buf[:nb] if rows is None else obs_buf.index_select(0, rows[:nb]))
+        v, a = self.dqn.heads(phi)
+        nn_ops.select_actions(v, a, rows, count, env.masks, env.row_table, env.row_step, env.row_seat, seed=self.seed,
+                              table_offset=table_offset, epsilon=self.boltzmann_epsilon, temp=self.boltzmann_temp, top_p=self.top_p,
+                              actions=actions, q_out=q_out, greedy=greedy)
+
+    @torch.inference_mode()
+    def decide(self, obs_buf, env, rows, count, n: int, *, table_offset: int, actions, q_out, greedy, bucket: int = 256):
+        """Decide batch rows i < n of the environment `env`: row rows[i] (rows None: i) of the persistent buffer obs_buf; `count` is
+        the same number as an int32 device tensor, which the captured graph reads at every replay. Writes actions, q_out and greedy
+        at the environment rows."""
+        nb = min((n + bucket - 1) // bucket * bucket, obs_buf.shape[0])
+        key = (obs_buf.data_ptr(), None if rows is None else rows.data_ptr(), count.data_ptr(), actions.data_ptr(), nb)
+        graph = self._graphs.get(key)
+        if graph is None:
+            args = (obs_buf, env, rows, count, nb, table_offset, actions, q_out, greedy)
+            cur = torch.cuda.current_stream(self.device)
+            side = torch.cuda.Stream(self.device)
+            side.wait_stream(cur)
+            with torch.cuda.stream(side):  # warm-up outside the capture (cuDNN algorithm selection, lazy init)
+                for _ in range(2):
+                    self._forward_select(*args)
+            cur.wait_stream(side)
+            graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(graph):
+                self._forward_select(*args)
+            self._graphs[key] = graph
+            self.graph_captures += 1
+        graph.replay()
+        self.graph_replays += 1

@@ -18,7 +18,10 @@ __profile__ = "release"
 __version__ = "0.1.0-mortal_b200"
 
 
-def install() -> None:
+def install(adopt_reference_engines: bool = False) -> None:
+    """With adopt_reference_engines, the arenas play MortalEngine objects (versions 2-4, not oracle, on the arena's CUDA device)
+    through mortal_b200.engine.ReferenceEngine on the device path instead of their react_batch; mortal/*.py stay unchanged."""
+    arena._Arena.adopt_reference_engines = bool(adopt_reference_engines)
     mod = sys.modules[__name__]
     sys.modules.setdefault("libriichi", mod)
     for sub in ("arena", "consts", "dataset", "stat", "state", "mjai"):

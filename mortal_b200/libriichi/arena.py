@@ -6,6 +6,10 @@ one_vs_three.rs:140-191 (game g = 4*s + r uses seed (seed_start[0] + s, seed_sta
 sits at absolute seat r). The step loop is BatchGame::run (game.rs:286-304) executed by mjx kernels;
 engines are called once per cycle per agent like MortalBatchAgent::evaluate (mortal.rs:114-159).
 
+With `adopt_reference_engines` (libriichi.install(adopt_reference_engines=True)), MortalEngine objects of versions 2-4 on the
+arena's device are played through mortal_b200.engine.ReferenceEngine: the observations never leave the GPU, the rows are split per
+agent on the device and each engine's forward + action selection replays as one CUDA graph, greedy or sampled, with or without logs.
+
 Tables are independent, so for reference-protocol engines (react_batch over host arrays) the batch is played as TWO half-batches
 stepped alternately (`pipeline`): while an engine works on the rows of one half on the host, the environment kernels and the
 D2H copies of the other half run. Results are those of one batch. Device engines run the batch as one.
@@ -16,14 +20,9 @@ import time
 
 import numpy as np
 
-from ..engine import HostProtocolEngine
+from ..engine import HostProtocolEngine, ReferenceEngine
 from ..env import BatchEnv
-
-
-def _adapt(engine):
-    if hasattr(engine, "react_device"):
-        return engine
-    return HostProtocolEngine(engine)
+from ..model import OBS_ROWS
 
 
 class _MetaRecorder:
@@ -53,8 +52,12 @@ class _MetaRecorder:
 
     @_guard
     def add_agent(self, cycle, idx, q, eval_ns, greedy=None):
+        """eval_ns: nanoseconds, or a (start, end) pair of CUDA events around the engine's work on the recording stream"""
         g = None if greedy is None else np.asarray(greedy.cpu() if hasattr(greedy, "cpu") else greedy, dtype=bool)
-        self.q.setdefault(cycle, []).append((idx.cpu().numpy(), q.float().cpu().numpy(), int(eval_ns), g))
+        entry = (idx.cpu().numpy(), q.float().cpu().numpy())  # synchronises the stream, so both events have completed
+        if isinstance(eval_ns, tuple):
+            eval_ns = max(1, int(eval_ns[0].elapsed_time(eval_ns[1]) * 1e6))
+        self.q.setdefault(cycle, []).append((*entry, int(eval_ns), g))
 
     @_guard
     def add_rows(self, cycle, tbl, row_seat, actions, masks, obs):
@@ -159,6 +162,17 @@ class _Part:
         if any(self.oracle) and self.host_mode:
             inv_rows = 211 if version == 1 else 217
             self.h_inv = pin(torch.empty((env.row_cap, inv_rows, 34), dtype=torch.float32))
+        # MortalEngines adopted onto the device path (ReferenceEngine): persistent per-version observation buffers (stable graph
+        # keys), the Q / greedy outputs of the select kernel, and for two engines the device-side split of the rows
+        self.adopted = all(isinstance(a, ReferenceEngine) for a in agents)
+        if self.adopted:
+            self.obs_bufs = {v: torch.empty((env.row_cap, OBS_ROWS[v], 34), dtype=torch.float32, device=dev) for v in set(versions)}
+            self.q_dev = self.q_all if self.q_all is not None else torch.zeros((env.row_cap, 46), dtype=torch.float32, device=dev)
+            self.greedy = torch.ones(env.row_cap, dtype=torch.uint8, device=dev)
+            if agents[0] is not agents[1]:  # agent 0 = challenger, 1 = champion
+                self.agent_of = torch.from_numpy((~self.ic_host[np.arange(self.n) % per]).astype(np.uint8)).to(dev)
+                self.split = [torch.zeros(env.row_cap, dtype=torch.int32, device=dev) for _ in range(2)]
+                self.counts = torch.zeros(2, dtype=torch.int32, device=dev)
         self.first, self.cycles, self.nr = True, 0, 0
         self.recorded, self.recorded_masks = [], []
         self.mask_weights = (1 << torch.arange(46, dtype=torch.int64))
@@ -262,6 +276,11 @@ class _Part:
                                                       h_actions[:nr].clone()], dim=1))
                     self.recorded_masks.append((self.h_masks[:nr].long() * self.mask_weights).sum(1))
                 return
+            if self.adopted:
+                obs = self._decide_adopted(nr, cycles, meta_rec)
+                if meta_rec is not None or self.arena.record_decisions:
+                    self._record(cycles, nr, env.row_table[:nr].long(), (env.row_seat[:nr] & 3).long(), env.masks[:nr], obs[:nr])
+                return
             obs_buf = env.encode_obs()
             obs, masks = obs_buf[:nr], env.masks[:nr]
             tbl = env.row_table[:nr].long()
@@ -299,12 +318,50 @@ class _Part:
                         self.q_all[idx] = q.float()
                     if meta_rec is not None:
                         meta_rec.add_agent(cycles, idx, q, time.perf_counter_ns() - t_eval)
-            if meta_rec is not None:
-                meta_rec.add_rows(cycles, tbl, env.row_seat[:nr], self.actions[:nr], masks, obs)
-            if self.arena.record_decisions:
-                self.recorded.append(torch.stack([tbl + self.offset, env.row_step[:nr].long(), seat, (env.row_seat[:nr] >> 2).long() & 1,
-                                                  self.actions[:nr]], dim=1).cpu())
-                self.recorded_masks.append((masks.long() * self.mask_weights.to(self.dev)).sum(1).cpu())
+            self._record(cycles, nr, tbl, seat, masks, obs)
+
+    def _decide_adopted(self, nr, cycles, meta_rec):
+        """ReferenceEngine agents: encode each obs version into its persistent buffer, split the rows per agent on the device (one
+        small read-back of the two counts), replay each engine's graph; the select kernel writes actions / Q / greedy in place."""
+        import torch
+
+        env, agents = self.env, self.agents
+        for v in (self.versions if self.mixed else self.versions[:1]):
+            if self.mixed:
+                env.set_obs_version(v)
+            env.encode_obs(out=self.obs_bufs[v])
+        if self.mixed:
+            env.set_obs_version(self.versions[0])
+        if agents[0] is agents[1]:
+            jobs = [(agents[0], None, env.n_rows_dev, nr, self.versions[0])]
+        else:
+            from .. import nn_ops
+
+            nn_ops.split_rows(env.row_table, env.row_seat, env.n_rows_dev, self.agent_of, self.split[0], self.split[1], self.counts)
+            counts = self.counts.tolist()
+            jobs = [(agents[k], self.split[k], self.counts[k:k + 1], counts[k], self.versions[k]) for k in range(2) if counts[k]]
+        for agent, rows, count, n, version in jobs:
+            ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) if meta_rec is not None else None
+            if ev:
+                ev[0].record()
+            agent.decide(self.obs_bufs[version], env, rows, count, n, table_offset=self.offset, actions=self.actions, q_out=self.q_dev,
+                         greedy=self.greedy)
+            if ev:
+                ev[1].record()
+                idx = torch.arange(n, device=self.dev) if rows is None else rows[:n].long()
+                meta_rec.add_agent(cycles, idx, self.q_dev[idx], ev, self.greedy[idx])
+        return self.obs_bufs[self.versions[0]]
+
+    def _record(self, cycles, nr, tbl, seat, masks, obs):
+        import torch
+
+        env, meta_rec = self.env, self.meta_rec
+        if meta_rec is not None:
+            meta_rec.add_rows(cycles, tbl, env.row_seat[:nr], self.actions[:nr], masks, obs)
+        if self.arena.record_decisions:
+            self.recorded.append(torch.stack([tbl + self.offset, env.row_step[:nr].long(), seat, (env.row_seat[:nr] >> 2).long() & 1,
+                                              self.actions[:nr]], dim=1).cpu())
+            self.recorded_masks.append((masks.long() * self.mask_weights.to(self.dev)).sum(1).cpu())
 
 
 class _RunState:
@@ -324,6 +381,7 @@ class _RunState:
 
 class _Arena:
     SEATS_PER_SEED = 4
+    adopt_reference_engines = False  # play eligible MortalEngines on the device path (ReferenceEngine); libriichi.install() sets it
 
     def __init__(self, *, disable_progress_bar: bool = False, log_dir=None, shuffle_kind: int = 0, device: int = 0):
         self.disable_progress_bar = disable_progress_bar
@@ -348,13 +406,26 @@ class _Arena:
     def _challenger_seats(self, game_in_seed: int):
         raise NotImplementedError
 
+    def _adapt(self, engine):
+        if hasattr(engine, "react_device"):
+            return engine
+        if self.adopt_reference_engines and ReferenceEngine.eligible(engine, self.device):
+            return ReferenceEngine(engine)
+        return HostProtocolEngine(engine)
+
     def _run(self, challenger, champion, seed_start, seed_count):
         import torch
 
         if challenger is champion:
-            agents = [_adapt(challenger)] * 2
+            agents = [self._adapt(challenger)] * 2
         else:
-            agents = [_adapt(challenger), _adapt(champion)]
+            agents = [self._adapt(challenger), self._adapt(champion)]
+        if not all(isinstance(a, ReferenceEngine) for a in agents):  # adoption covers both agents or neither
+            agents = [HostProtocolEngine(a.engine) if isinstance(a, ReferenceEngine) else a for a in agents]
+        for a in {id(a): a for a in agents}.values():
+            if isinstance(a, ReferenceEngine):
+                a.refresh()
+        self.last_agents = agents
         for a in agents:
             if getattr(a, "version", 4) not in (1, 2, 3, 4):
                 raise ValueError(f"unsupported obs version {a.version} (consts.rs:18 MAX_VERSION = 4)")

@@ -1,10 +1,11 @@
 """Policy/value network used by the benchmark and examples (stays ordinary PyTorch, as north_star asks).
 
-Architecture restated from mortal/model.py:10-231 (version 4): Conv1d stem -> `num_blocks` pre-activation
+Architecture restated from mortal/model.py:10-231 (versions 2-4): Conv1d stem -> `num_blocks` pre-activation
 residual blocks (BN -> Mish -> Conv1d k3, twice) each gated by a squeeze/excite style channel attention
--> BN -> Mish -> Conv1d(C, 32, k3) -> Mish -> Linear(32*34, 1024) -> Mish ; dueling head Linear(1024, 1+46)
-with the advantage mean taken over legal actions only and illegal actions at -inf. Real Mortal checkpoints
-load into mortal/model.py unchanged; this module exists so bench.py does not depend on /root/reference.
+-> BN -> Mish -> Conv1d(C, 32, k3) -> Mish -> Linear(32*34, 1024) -> Mish ; dueling head Linear(1024, 1+46) (v4) or
+two Linear -> Mish -> Linear MLPs (v2: hidden 512, v3: 256) with the advantage mean taken over legal actions only and illegal
+actions at -inf. Versions differ in the stem's input rows and the BatchNorm eps (v2 1e-5, v3/v4 1e-3). Mortal checkpoints load
+through mortal_b200.checkpoint.
 """
 from __future__ import annotations
 
@@ -13,6 +14,13 @@ from torch import nn
 
 OBS_ROWS = {1: 938, 2: 942, 3: 934, 4: 1012}  # consts.rs:20-28
 ACTION_SPACE = 46
+BN_EPS = {2: 1e-5, 3: 1e-3, 4: 1e-3}  # not stored in a state_dict: the versions' BatchNorm1d constructors differ
+DQN_HIDDEN = {2: 512, 3: 256}
+
+
+def _check_version(version: int):
+    if version not in BN_EPS:
+        raise ValueError(f"network version {version} is not supported (2, 3 or 4)")
 
 
 class ChannelGate(nn.Module):
@@ -38,11 +46,11 @@ class ChannelGate(nn.Module):
 
 
 class PreActBlock(nn.Module):
-    def __init__(self, channels: int):
+    def __init__(self, channels: int, eps: float = 1e-3):
         super().__init__()
-        self.bn1 = nn.BatchNorm1d(channels, momentum=0.01, eps=1e-3)
+        self.bn1 = nn.BatchNorm1d(channels, momentum=0.01, eps=eps)
         self.conv1 = nn.Conv1d(channels, channels, 3, padding=1, bias=False)
-        self.bn2 = nn.BatchNorm1d(channels, momentum=0.01, eps=1e-3)
+        self.bn2 = nn.BatchNorm1d(channels, momentum=0.01, eps=eps)
         self.conv2 = nn.Conv1d(channels, channels, 3, padding=1, bias=False)
         self.act = nn.Mish(inplace=True)
         self.gate = ChannelGate(channels)
@@ -81,12 +89,12 @@ class PreActBlock(nn.Module):
 class Brain(nn.Module):
     def __init__(self, *, conv_channels: int = 192, num_blocks: int = 40, version: int = 4):
         super().__init__()
-        assert version == 4, "only the version-4 network is restated here"
+        _check_version(version)
         self.version = version
-        c = conv_channels
+        c, eps = conv_channels, BN_EPS[version]
         self.stem = nn.Conv1d(OBS_ROWS[version], c, 3, padding=1, bias=False)
-        self.blocks = nn.Sequential(*[PreActBlock(c) for _ in range(num_blocks)])
-        self.bn = nn.BatchNorm1d(c, momentum=0.01, eps=1e-3)
+        self.blocks = nn.Sequential(*[PreActBlock(c, eps) for _ in range(num_blocks)])
+        self.bn = nn.BatchNorm1d(c, momentum=0.01, eps=eps)
         self.act = nn.Mish(inplace=True)
         self.neck = nn.Conv1d(c, 32, 3, padding=1)
         self.fc = nn.Linear(32 * 34, 1024)
@@ -132,12 +140,19 @@ class Brain(nn.Module):
         if fused and obs.dtype == torch.float32 and obs.is_contiguous():
             from . import nn_ops
 
-            x = F.conv2d(nn_ops.obs_to_nhwc(obs, self._cpad), self._w_stem_pad, padding=(0, 1))
-        else:
-            if self._fast_dtype is not None:
-                obs = obs.to(self._fast_dtype)
-            x = obs.unsqueeze(2).contiguous(memory_format=torch.channels_last)  # [B, C, 1, 34]
-            x = F.conv2d(x, self._w_stem, padding=(0, 1))
+            return self.forward_fast_nhwc(nn_ops.obs_to_nhwc(obs, self._cpad))
+        if self._fast_dtype is not None:
+            obs = obs.to(self._fast_dtype)
+        x = obs.unsqueeze(2).contiguous(memory_format=torch.channels_last)  # [B, C, 1, 34]
+        return self._trunk_fast(F.conv2d(x, self._w_stem, padding=(0, 1)))
+
+    def forward_fast_nhwc(self, x):
+        """forward_fast from the stem input already in the padded bf16 channels-last layout nn_ops.obs_to_nhwc emits"""
+        return self._trunk_fast(torch.nn.functional.conv2d(x, self._w_stem_pad, padding=(0, 1)))
+
+    def _trunk_fast(self, x):
+        F = torch.nn.functional
+        fused = x.is_cuda and self._fast_dtype == torch.bfloat16
         if fused:
             # libmjx kernels (csrc/mjx_nn.cuh) around the cuDNN convolutions: per block one BN-affine+Mish pass and one pass for
             # everything between conv2 and the next block's conv1 (pooling, gate MLP, sigmoid, gate * y + x, next BN-affine+Mish)
@@ -164,11 +179,23 @@ class Brain(nn.Module):
 class DQN(nn.Module):
     def __init__(self, *, version: int = 4):
         super().__init__()
-        assert version == 4
-        self.net = nn.Linear(1024, 1 + ACTION_SPACE)
-        nn.init.zeros_(self.net.bias)
+        _check_version(version)
+        self.version = version
+        if version == 4:
+            self.net = nn.Linear(1024, 1 + ACTION_SPACE)
+            nn.init.zeros_(self.net.bias)
+        else:
+            h = DQN_HIDDEN[version]
+            self.v_head = nn.Sequential(nn.Linear(1024, h), nn.Mish(inplace=True), nn.Linear(h, 1))
+            self.a_head = nn.Sequential(nn.Linear(1024, h), nn.Mish(inplace=True), nn.Linear(h, ACTION_SPACE))
+
+    def heads(self, phi):
+        """(value [B, 1], advantage [B, 46]) before the masked dueling combination"""
+        if self.version == 4:
+            return self.net(phi).split((1, ACTION_SPACE), dim=-1)
+        return self.v_head(phi), self.a_head(phi)
 
     def forward(self, phi, mask):
-        v, a = self.net(phi).split((1, ACTION_SPACE), dim=-1)
+        v, a = self.heads(phi)
         a_mean = a.masked_fill(~mask, 0.0).sum(-1, keepdim=True) / mask.sum(-1, keepdim=True)
         return (v + a - a_mean).masked_fill(~mask, -torch.inf)

@@ -7,6 +7,9 @@ Runs in the dev container (needs /root/reference). Outputs are committed:
   tests/golden/golden_game.jsonl — the seeded full-game log embedded in log-viewer/index.example.html:10-264
   tests/golden/ref_tables.json — libriichi's shanten / agari data files (algo/data/*.bin.gz) as a digest of their whole
       content plus a seeded sample of rows / keys (tests/test_tables.py compares the generated tables against both)
+  tests/golden/ref_model_outputs.json — for network versions 2-4 at 32 channels x 2 blocks: the key schema of mortal/model.py's
+      Brain / DQN state_dicts, the seeds of tests/ref_checkpoint_fixture.py's weights and inputs, and the Q-values Mortal's
+      modules compute from them (fp32, CPU); tests/test_reference_checkpoint.py loads the same weights into mortal_b200
 """
 import gzip
 import hashlib
@@ -50,8 +53,57 @@ def table_fixtures() -> dict:
     return out
 
 
+def model_fixtures() -> dict:
+    """Mortal's own Brain / DQN (mortal/model.py) on seeded weights and inputs, fp32 on the CPU: the key schema of each
+    version's state_dicts and the Q-values for tests/ref_checkpoint_fixture.py's inputs. Data only."""
+    import importlib.util
+    import types
+
+    import torch
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    sys.path.insert(0, root)
+    sys.path.insert(0, os.path.join(root, "tests"))
+    import ref_checkpoint_fixture as F
+    from mortal_b200.libriichi import consts
+
+    # mortal/model.py imports only obs_shape / oracle_obs_shape / ACTION_SPACE / GRP_SIZE from libriichi.consts
+    pkg = types.ModuleType("libriichi")
+    pkg.consts = consts
+    sys.modules.setdefault("libriichi", pkg)
+    sys.modules.setdefault("libriichi.consts", consts)
+    spec = importlib.util.spec_from_file_location("mortal_reference_model", os.path.join(REF, "mortal/model.py"))
+    model = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(model)
+    torch.set_num_threads(4)
+    out = {"channels": F.CHANNELS, "blocks": F.BLOCKS, "rows": F.ROWS, "versions": {}}
+    for version in F.VERSIONS:
+        brain = model.Brain(conv_channels=F.CHANNELS, num_blocks=F.BLOCKS, version=version)
+        dqn = model.DQN(version=version)
+        strip = lambda sd: {k: tuple(v.shape) for k, v in sd.items() if not k.endswith("num_batches_tracked")}
+        schema = (strip(brain.state_dict()), strip(dqn.state_dict()))
+        weight_seed, input_seed = 7000 + version, 8000 + version
+        bsd, dsd = F.make_state_dicts(schema, weight_seed)
+        brain.load_state_dict({k: torch.from_numpy(v) for k, v in bsd.items()}, strict=False)
+        dqn.load_state_dict({k: torch.from_numpy(v) for k, v in dsd.items()})
+        brain.eval(), dqn.eval()
+        obs, masks = F.make_inputs(version, F.ROWS, input_seed)
+        with torch.no_grad():
+            q = dqn(brain(torch.from_numpy(obs)), torch.from_numpy(masks)).double().numpy()
+        out["versions"][str(version)] = {
+            "brain_schema": [[k, list(s)] for k, s in schema[0].items()],
+            "dqn_schema": [[k, list(s)] for k, s in schema[1].items()],
+            "weight_seed": weight_seed, "input_seed": input_seed,
+            "q": [[None if np.isneginf(x) else float(x) for x in row] for row in q],
+        }
+    return out
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
+    with open(os.path.join(OUT, "ref_model_outputs.json"), "w") as f:
+        json.dump(model_fixtures(), f)
+        f.write("\n")
     src = open(os.path.join(REF, "libriichi/src/state/test.rs")).read()
     logs = {}
     cur = None
